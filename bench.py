@@ -41,7 +41,15 @@ def parse():
     ap.add_argument("--dtype", default=os.environ.get("GG_BENCH_DTYPE", "f32"), choices=["f32", "bf16"],
                     help="activation storage type: f32 = BASELINE config 2 (the headline), bf16 = config 3")
     ap.add_argument("--no-extra", action="store_true", help="skip the additional config-3 (bf16) measurement of the default run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy; the run then uses cuDNN's deterministic "
+                         "algorithms (config.cudnn in the result line), so that the same arguments give the same files")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -102,7 +110,8 @@ def workload_config(args, dtype="f32"):
             "step_mode": "eager" if args.no_graph else "whole-step CUDA graph replay",
             "per_gpu_batch": args.batch, "global_batch": args.batch * args.gpus, "gen_size": 256, "flow_size": 128,
             "parallelism": "dp%d" % args.gpus, "activation_layout": "NHWC (channels-last) generator + STN trunk",
-            "l2_policy": "inputs larger than L2 (activations of one step >> 126 MB)"}
+            "l2_policy": "inputs larger than L2 (activations of one step >> 126 MB)",
+            "cudnn": "deterministic (heuristic choice)" if args.dump_outputs else "benchmark (timed choice)"}
 
 
 # --------------------------------------------------------------------------------------------------- reference arm
@@ -166,7 +175,24 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------------------------------- our arm
-def measure(args, dtype, dev, rank, world, distributed, want_clocks):
+DUMP_SAMPLE = 1 << 20   # parameters kept per module by snapshot(): 4 MB of float32 each
+
+
+def snapshot(tr, out):
+    """What the last timed step computed, copied to the host: the losses step() returned and the STN's parameters and their
+    EMA after its optimiser update -- all of them, or a fixed, seeded sample of DUMP_SAMPLE elements (the same positions in
+    every run of the same configuration)."""
+    arrays = {"loss_" + k: v.detach().double().cpu().numpy().reshape(-1) for k, v in out.items()}
+    for name, module in (("stn_params", tr.t_module), ("stn_ema_params", tr.t_ema)):
+        flat = torch.cat([p.detach().float().reshape(-1) for p in module.parameters()])
+        if flat.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            flat = flat[idx.to(flat.device)]
+        arrays[name] = flat.cpu().numpy()
+    return arrays
+
+
+def measure(args, dtype, dev, rank, world, distributed, want_clocks, want_outputs=False):
     """Build the trainer for `dtype`, warm up, probe the roofline kernel, capture the step, time `args.steps` steps twice
     (device-resident latents; end to end with host latents) -> dict of raw measurements (max over ranks)."""
     import torch.distributed as dist
@@ -230,6 +256,7 @@ def measure(args, dtype, dev, rank, world, distributed, want_clocks):
         torch.cuda.cudart().cudaProfilerStop()
     ms = st.elapsed_time(en)
     phase("timed region 1 done")
+    outputs = snapshot(tr, out) if want_outputs else None
     if sampler:
         sampler.stop_flag.set()
 
@@ -252,7 +279,7 @@ def measure(args, dtype, dev, rank, world, distributed, want_clocks):
     if distributed:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms, ms2 = t.tolist()
-    return {"tr": tr, "cfg": cfg, "ms": ms, "ms2": ms2, "timing": timing, "calls": calls_per_step * args.steps,
+    return {"tr": tr, "cfg": cfg, "ms": ms, "ms2": ms2, "timing": timing, "calls": calls_per_step * args.steps, "outputs": outputs,
             "clocks": sampler.summary() if sampler else None, "losses": {k: float(v.detach()) for k, v in out.items()}}
 
 
@@ -302,10 +329,15 @@ def run_ours(args):
     torch.cuda.set_device(local_rank)
     dev = "cuda:%d" % local_rank
     rank = gdist.get_rank()
-    torch.backends.cudnn.benchmark = True
+    # a dump must be the same on every run with the same arguments: cuDNN's timed algorithm choice can differ from run to
+    # run, and the training step carries any difference forward through Adam -- so a dumping run takes its heuristic
+    # choice of deterministic algorithms (config.cudnn says which mode the timed numbers were measured in)
+    torch.backends.cudnn.benchmark = not args.dump_outputs
+    torch.backends.cudnn.deterministic = bool(args.dump_outputs)
     phase("process group ready (world %d)" % world)
 
-    m = measure(args, args.dtype, dev, rank, world, distributed, want_clocks=True)
+    m = measure(args, args.dtype, dev, rank, world, distributed, want_clocks=True,
+                want_outputs=bool(args.dump_outputs) and rank == 0)
     images = args.batch * world * args.steps
     extra = None
     other = "bf16" if args.dtype == "f32" else None
@@ -358,6 +390,11 @@ def run_ours(args):
             "clocks": m["clocks"], "losses": m["losses"]}
     if extra is not None:
         line["config3_bf16"] = extra
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, array in m["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), array)
     print(json.dumps(line), flush=True)
     phase("result printed")
     finish(distributed, tr)

@@ -72,8 +72,10 @@ SIGNATURES = {
     "gg_splat2d_workspace": (_L, [_L, _I, _I, _I]),
     "gg_splat2d_forward": (_I, [_P] * 6 + [_L, _L, _I, _I, _I, _I, _P]),
     "gg_flow_compose_forward": (_I, [_P] * 7 + [_L, _I, _I, _I, _P]),
-    "gg_flow_compose_backward": (_I, [_P] * 10 + [_L, _I, _I, _I, _P]),
-    "gg_mipmap_warp_backward": (_I, [_P] * 7 + [_I, _L] + [_I] * 6 + [_F, _F, _I, _P]),
+    "gg_flow_compose_backward_workspace": (_L, [_L, _I, _I, _I]),
+    "gg_flow_compose_backward": (_I, [_P] * 11 + [_L, _I, _I, _I, _P]),
+    "gg_mipmap_warp_backward_workspace": (_L, [_L, _I, _I]),
+    "gg_mipmap_warp_backward": (_I, [_P] * 8 + [_I, _L] + [_I] * 6 + [_F, _F, _I, _P]),
 }
 
 _dll = None
@@ -201,6 +203,11 @@ def invalidate(t):
         t._gg_cache = None
     except Exception:
         pass
+
+
+def workspace(nbytes, device):
+    """A device scratch buffer of at least `nbytes` bytes from PyTorch's caching allocator (which aligns blocks to 512 B)."""
+    return torch.empty(max(1, (int(nbytes) + 3) // 4), dtype=torch.float32, device=device)
 
 
 def stream():

@@ -82,10 +82,12 @@ flow_compose_fwd_kernel(float* __restrict__ delta_out, float* __restrict__ flow_
   }
 }
 
-// backward: g_delta (direct, may be null) and g_flow (may be null) -> g_mask (written), g_low (atomics, zeroed by
-// caller), g_base (atomics, zeroed by caller)
+// backward: g_delta (direct, may be null) and g_flow (may be null) -> g_mask (written); the per-pixel terms of g_low
+// (one per tap) and of g_base (6 per pixel) go to the caller's workspace, and flow_low_gather_kernel /
+// flow_base_reduce_kernel sum them in a fixed order (no float atomics: the same bits on every run).  The g_low terms are
+// laid out by the low-res cell they belong to, (N, H, W, 9, S, S): each cell's terms are contiguous.
 __global__ void __launch_bounds__(256)
-flow_compose_bwd_kernel(float* __restrict__ g_mask, float* __restrict__ g_low, float* __restrict__ g_base,
+flow_compose_bwd_kernel(float* __restrict__ g_mask, float2* __restrict__ g_low, float* __restrict__ g_base,
                         const float* __restrict__ g_delta, const float* __restrict__ g_flow,
                         const float* __restrict__ low, const float* __restrict__ mask,
                         const float* __restrict__ identity, const float* __restrict__ base,
@@ -129,21 +131,9 @@ flow_compose_bwd_kernel(float* __restrict__ g_mask, float* __restrict__ g_low, f
         const float gx = id.x + dx, gy = id.y + dy;
         const float* M = base + n * 6;
         if (g_base) {
-          float* gb = g_base + n * 6;
-          // block-level pre-reduction would need uniform n per block; tensors are tiny -> warp-aggregate then atomics
-          float v[6] = {gf.x * gx, gf.x * gy, gf.x, gf.y * gx, gf.y * gy, gf.y};
-          const unsigned act = __activemask();
-          const int64_t n_lead = __shfl_sync(act, n, __ffs(act) - 1);
-          if (act == 0xffffffffu && __all_sync(act, n == n_lead)) {  // whole warp in one sample: 6 atomics per warp
-#pragma unroll
-            for (int q = 0; q < 6; ++q) {
-              const float r = warp_sum(v[q]);
-              if ((threadIdx.x & 31) == 0) atomicAdd(gb + q, r);
-            }
-          } else {
-#pragma unroll
-            for (int q = 0; q < 6; ++q) atomicAdd(gb + q, v[q]);
-          }
+          float* gb = g_base + idx * 6;
+          gb[0] = gf.x * gx; gb[1] = gf.x * gy; gb[2] = gf.x;
+          gb[3] = gf.y * gx; gb[4] = gf.y * gy; gb[5] = gf.y;
         }
         const float px = M[0] * gf.x + M[3] * gf.y;
         const float py = M[1] * gf.x + M[4] * gf.y;
@@ -161,14 +151,62 @@ flow_compose_bwd_kernel(float* __restrict__ g_mask, float* __restrict__ g_low, f
       if (g_low) {
         const int hh = h + k / 3 - 1, ww = w + k % 3 - 1;
         if (hh >= 0 && hh < p.h && ww >= 0 && ww < p.w) {
-          float* gl = g_low + ((n * p.h + hh) * static_cast<int64_t>(p.w) + ww) * 2;
           const float sc = static_cast<float>(p.s) * pk[k];
-          atomicAdd(gl + 0, sc * gdx);
-          atomicAdd(gl + 1, sc * gdy);
+          const int64_t cell = (n * p.h + hh) * static_cast<int64_t>(p.w) + ww;
+          g_low[((cell * 9 + k) * p.s + sy) * p.s + sx] = make_float2(sc * gdx, sc * gdy);
         }
       }
     }
   }
+}
+
+// g_low[n, hh, ww] = sum of the 9*S*S terms of low-res cell (hh, ww) (taps whose source cell is outside the grid have
+// none): one warp per cell, coalesced reads, lane-strided sums and a shuffle tree -- a fixed order
+__global__ void __launch_bounds__(256)
+flow_low_gather_kernel(float* __restrict__ g_low, const float2* __restrict__ terms, FlowParams p, int64_t cells) {
+  const int lane = threadIdx.x & 31;
+  const int ss = p.s * p.s;
+  for (int64_t c = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; c < cells;
+       c += (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5) {
+    const int ww = static_cast<int>(c % p.w);
+    const int hh = static_cast<int>((c / p.w) % p.h);
+    const float2* t = terms + c * 9 * ss;
+    float gx = 0.f, gy = 0.f;
+    for (int e = lane; e < 9 * ss; e += 32) {
+      const int k = e / ss;
+      const int h = hh - (k / 3 - 1), w = ww - (k % 3 - 1);
+      if (h < 0 || h >= p.h || w < 0 || w >= p.w) continue;
+      const float2 v = t[e];
+      gx += v.x; gy += v.y;
+    }
+    gx = warp_sum(gx);
+    gy = warp_sum(gy);
+    if (lane == 0) *reinterpret_cast<float2*>(g_low + c * 2) = make_float2(gx, gy);
+  }
+}
+
+// g_base[n, q] = sum of the 6 per-pixel terms over sample n: one block per sample, fixed-order tree reduction
+__global__ void __launch_bounds__(256)
+flow_base_reduce_kernel(float* __restrict__ g_base, const float* __restrict__ terms, int64_t per_sample) {
+  __shared__ float red[6][256];
+  const int64_t n = blockIdx.x;
+  float acc[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  for (int64_t i = threadIdx.x; i < per_sample; i += blockDim.x) {
+    const float* t = terms + (n * per_sample + i) * 6;
+#pragma unroll
+    for (int q = 0; q < 6; ++q) acc[q] += t[q];
+  }
+#pragma unroll
+  for (int q = 0; q < 6; ++q) red[q][threadIdx.x] = acc[q];
+  __syncthreads();
+  for (int half = blockDim.x / 2; half > 0; half >>= 1) {
+    if (threadIdx.x < half) {
+#pragma unroll
+      for (int q = 0; q < 6; ++q) red[q][threadIdx.x] += red[q][threadIdx.x + half];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x < 6) g_base[n * 6 + threadIdx.x] = red[threadIdx.x][0];
 }
 
 inline int flow_grid(int64_t total) {
@@ -199,8 +237,13 @@ int gg_flow_compose_forward(float* delta_flow, float* flow, const float* low_flo
   return GG_OK;
 }
 
-int gg_flow_compose_backward(float* grad_mask, float* grad_low_flow, float* grad_base_warp, const float* grad_delta,
-                             const float* grad_flow, const float* low_flow, const float* mask,
+int64_t gg_flow_compose_backward_workspace(int64_t N, int H, int W, int S) {
+  const int64_t pixels = N * S * S * H * static_cast<int64_t>(W);
+  return pixels * 9 * static_cast<int64_t>(sizeof(float2)) + pixels * 6 * static_cast<int64_t>(sizeof(float));
+}
+
+int gg_flow_compose_backward(float* grad_mask, float* grad_low_flow, float* grad_base_warp, void* workspace,
+                             const float* grad_delta, const float* grad_flow, const float* low_flow, const float* mask,
                              const float* identity_flow, const float* base_warp, const float* alpha, int64_t N,
                              int H, int W, int S, void* stream) {
   if (N < 0 || H < 1 || W < 1 || S < 1) return fail(GG_ERR_BAD_ARG, "flow_compose_backward: bad shape");
@@ -209,10 +252,30 @@ int gg_flow_compose_backward(float* grad_mask, float* grad_low_flow, float* grad
   if (grad_flow && base_warp && !identity_flow) return fail(GG_ERR_BAD_ARG, "flow_compose_backward: identity_flow required");
   FlowParams p{N, H, W, S};
   const int64_t total = N * S * S * H * static_cast<int64_t>(W);
-  flow_compose_bwd_kernel<<<flow_grid(total), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      grad_mask, grad_low_flow, grad_base_warp, grad_delta, grad_flow, low_flow, mask, identity_flow, base_warp, alpha,
+  if ((grad_low_flow || grad_base_warp) && !workspace)
+    return fail(GG_ERR_BAD_ARG, "flow_compose_backward: grad_low_flow / grad_base_warp need a workspace");
+  auto st = static_cast<cudaStream_t>(stream);
+  // both outputs are written in full (the caller need not zero them)
+  float2* low_terms = grad_low_flow ? static_cast<float2*>(workspace) : nullptr;
+  float* base_terms = (grad_base_warp && grad_flow && base_warp)
+                          ? reinterpret_cast<float*>(static_cast<char*>(workspace) + total * 9 * sizeof(float2)) : nullptr;
+  if (grad_base_warp && !base_terms) {
+    if (cudaMemsetAsync(grad_base_warp, 0, N * 6 * sizeof(float), st) != cudaSuccess)
+      return fail(GG_ERR_CUDA, "flow_compose_backward: memset failed");
+  }
+  flow_compose_bwd_kernel<<<flow_grid(total), 256, 0, st>>>(
+      grad_mask, low_terms, base_terms, grad_delta, grad_flow, low_flow, mask, identity_flow, base_warp, alpha,
       p, total);
   GG_CHECK_LAUNCH("flow_compose_bwd launch");
+  if (low_terms) {
+    const int64_t cells = N * H * static_cast<int64_t>(W);
+    flow_low_gather_kernel<<<flow_grid(cells * 32), 256, 0, st>>>(grad_low_flow, low_terms, p, cells);
+    GG_CHECK_LAUNCH("flow_low_gather launch");
+  }
+  if (base_terms) {
+    flow_base_reduce_kernel<<<static_cast<unsigned>(N), 256, 0, st>>>(grad_base_warp, base_terms, total / N);
+    GG_CHECK_LAUNCH("flow_base_reduce launch");
+  }
   return GG_OK;
 }
 

@@ -575,11 +575,20 @@ __device__ __forceinline__ void scatter_level(float* __restrict__ grad_src, floa
     }
 }
 
+// the level-of-detail part of a grid pixel's gradient that belongs to the neighbour `target` (-1: none)
+struct NbGrad {
+  float x, y;
+  int target, pad;
+};
+
+// grad_grid (written in full): each pixel stores its own part; with MIP the part owed to a neighbour goes to `nb` (the
+// caller's workspace), and warp_grid_gather_kernel adds it in a fixed order (no float atomics: the same bits on every run)
 template <typename T, bool MIP>
 __global__ void __launch_bounds__(256)
 warp_bwd_kernel(float* __restrict__ grad_src, float* __restrict__ grad_pyr, float* __restrict__ grad_grid,
-                const T* __restrict__ grad_out, const T* __restrict__ src, const float* __restrict__ pyr,
-                const float* __restrict__ grid, const __grid_constant__ WarpParams p, int64_t total) {
+                NbGrad* __restrict__ nb, const T* __restrict__ grad_out, const T* __restrict__ src,
+                const float* __restrict__ pyr, const float* __restrict__ grid, const __grid_constant__ WarpParams p,
+                int64_t total) {
   for (int64_t idx = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; idx < total;
        idx += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int ox = static_cast<int>(idx % p.wo);
@@ -622,6 +631,7 @@ warp_bwd_kernel(float* __restrict__ grad_src, float* __restrict__ grad_pyr, floa
     if (grad_grid) {
       float* gg_n = grad_grid + grid_off;
       float ax = gix * s.mx, ay = giy * s.my;
+      NbGrad out_nb{0.f, 0.f, -1, 0};
       if (MIP && li.pass && glevel != 0.f && li.sq_arg >= 1.f) {
         // level = log2(dmax); dmax = sqrt(sq) of the arg-max neighbour (clamp(min=1) passes: sq >= 1)
         const float g_sq = glevel / (li.dmax * 0.6931471805599453f) * (0.5f / li.dmax);
@@ -629,13 +639,37 @@ warp_bwd_kernel(float* __restrict__ grad_src, float* __restrict__ grad_pyr, floa
         const float gox = 2.f * li.dx * g_sq * sx, goy = 2.f * li.dy * g_sq * sy;
         const int ny = (li.arg == 2) ? max(oy - 1, 0) : (li.arg == 3 ? min(oy + 1, p.ho - 1) : oy);
         const int nx = (li.arg == 0) ? max(ox - 1, 0) : (li.arg == 1 ? min(ox + 1, p.wo - 1) : ox);
-        atomicAdd(gg_n + (static_cast<int64_t>(ny) * p.wo + nx) * 2 + 0, gox);
-        atomicAdd(gg_n + (static_cast<int64_t>(ny) * p.wo + nx) * 2 + 1, goy);
+        out_nb = NbGrad{gox, goy, ny * p.wo + nx, 0};
         ax -= gox; ay -= goy;
       }
-      atomicAdd(gg_n + (static_cast<int64_t>(oy) * p.wo + ox) * 2 + 0, ax);
-      atomicAdd(gg_n + (static_cast<int64_t>(oy) * p.wo + ox) * 2 + 1, ay);
+      *reinterpret_cast<float2*>(gg_n + (static_cast<int64_t>(oy) * p.wo + ox) * 2) = make_float2(ax, ay);
+      if (MIP) nb[idx] = out_nb;
     }
+  }
+}
+
+// grad_grid[pixel] += the parts its neighbours (and, clamped at a border, itself) owe it, in a fixed order
+__global__ void __launch_bounds__(256)
+warp_grid_gather_kernel(float* __restrict__ grad_grid, const NbGrad* __restrict__ nb, int ho, int wo, int64_t total) {
+  for (int64_t idx = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; idx < total;
+       idx += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int ox = static_cast<int>(idx % wo);
+    const int oy = static_cast<int>((idx / wo) % ho);
+    const int me = oy * wo + ox;
+    const int64_t base = idx - me;
+    float gx = 0.f, gy = 0.f;
+    const int dy[5] = {0, 0, 0, -1, 1}, dx[5] = {0, -1, 1, 0, 0};
+#pragma unroll
+    for (int q = 0; q < 5; ++q) {
+      const int y = oy + dy[q], x = ox + dx[q];
+      if (y < 0 || y >= ho || x < 0 || x >= wo) continue;
+      const NbGrad v = nb[base + y * wo + x];
+      if (v.target == me) { gx += v.x; gy += v.y; }
+    }
+    float2* g = reinterpret_cast<float2*>(grad_grid + idx * 2);
+    float2 cur = *g;
+    cur.x += gx; cur.y += gy;
+    *g = cur;
   }
 }
 
@@ -838,7 +872,11 @@ int gg_stn_sample_forward(void* out, float* grid_out, float* delta_out, float* l
   return GG_OK;
 }
 
-int gg_mipmap_warp_backward(float* grad_src, float* grad_pyramid, float* grad_grid, const void* grad_out,
+int64_t gg_mipmap_warp_backward_workspace(int64_t N, int ho, int wo) {
+  return N * ho * static_cast<int64_t>(wo) * static_cast<int64_t>(sizeof(NbGrad));
+}
+
+int gg_mipmap_warp_backward(float* grad_src, float* grad_pyramid, float* grad_grid, void* workspace, const void* grad_out,
                             const void* src, const float* pyramid, const float* grid, int dtype, int64_t N, int C,
                             int hs, int ws, int ho, int wo, int extra_levels, float max_level, float min_level,
                             int padding_mode, void* stream) {
@@ -852,12 +890,14 @@ int gg_mipmap_warp_backward(float* grad_src, float* grad_pyramid, float* grad_gr
   if (!grad_src && !grad_grid) return GG_OK;
   auto st = static_cast<cudaStream_t>(stream);
   const int gridsz = grid_for(total, 256);
+  NbGrad* nb = (grad_grid && extra_levels > 0) ? static_cast<NbGrad*>(workspace) : nullptr;
+  if (grad_grid && extra_levels > 0 && !nb) return fail(GG_ERR_BAD_ARG, "mipmap_warp_backward: grad_grid needs a workspace");
 #define GG_BWD(T_)                                                                                               \
   if (extra_levels > 0)                                                                                          \
-    warp_bwd_kernel<T_, true><<<gridsz, 256, 0, st>>>(grad_src, grad_pyramid, grad_grid,                        \
+    warp_bwd_kernel<T_, true><<<gridsz, 256, 0, st>>>(grad_src, grad_pyramid, grad_grid, nb,                    \
         static_cast<const T_*>(grad_out), static_cast<const T_*>(src), pyramid, grid, wp, total);               \
   else                                                                                                           \
-    warp_bwd_kernel<T_, false><<<gridsz, 256, 0, st>>>(grad_src, grad_pyramid, grad_grid,                       \
+    warp_bwd_kernel<T_, false><<<gridsz, 256, 0, st>>>(grad_src, grad_pyramid, grad_grid, nb,                   \
         static_cast<const T_*>(grad_out), static_cast<const T_*>(src), pyramid, grid, wp, total)
   switch (dtype) {
     case GG_F32: GG_BWD(float); break;
@@ -867,6 +907,10 @@ int gg_mipmap_warp_backward(float* grad_src, float* grad_pyramid, float* grad_gr
   }
 #undef GG_BWD
   GG_CHECK_LAUNCH("warp_bwd launch");
+  if (nb) {
+    warp_grid_gather_kernel<<<gridsz, 256, 0, st>>>(grad_grid, nb, ho, wo, total);
+    GG_CHECK_LAUNCH("warp_grid_gather launch");
+  }
   return GG_OK;
 }
 

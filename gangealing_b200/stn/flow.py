@@ -65,9 +65,10 @@ class _FlowCompose(Function):
         g_delta = _f32c(g_delta) if g_delta is not None else None
         g_flow = _f32c(g_flow) if (g_flow is not None and g_flow.dim() == 4) else None
         g_mask = torch.empty_like(mask) if need_mask else None
-        g_low = torch.zeros_like(low) if need_low else None
-        g_base = torch.zeros((n, 2, 3), dtype=torch.float32, device=low.device) if (need_base and base is not None) else None
-        rc = _lib.load().gg_flow_compose_backward(_lib.ptr(g_mask), _lib.ptr(g_low), _lib.ptr(g_base), _lib.ptr(g_delta),
+        g_low = torch.empty_like(low) if need_low else None
+        g_base = torch.empty((n, 2, 3), dtype=torch.float32, device=low.device) if (need_base and base is not None) else None
+        scratch = _lib.workspace(_lib.load().gg_flow_compose_backward_workspace(n, h, w, s), low.device) if (g_low is not None or g_base is not None) else None
+        rc = _lib.load().gg_flow_compose_backward(_lib.ptr(g_mask), _lib.ptr(g_low), _lib.ptr(g_base), _lib.ptr(scratch), _lib.ptr(g_delta),
                                                   _lib.ptr(g_flow), low.data_ptr(), mask.data_ptr(), _lib.ptr(ident),
                                                   _lib.ptr(base), _lib.ptr(alpha), n, h, w, s, _lib.stream())
         _lib.check(rc, "gg_flow_compose_backward")

@@ -76,8 +76,9 @@ class _MipmapWarp(Function):
             go = go.to(x.dtype)
         grad_src = torch.zeros(x.shape, dtype=torch.float32, device=x.device) if need_x else None
         grad_pyr = torch.zeros_like(pyr) if (need_x and pyr is not None) else None
-        grad_grid = torch.zeros(g.shape, dtype=torch.float32, device=x.device) if need_g else None
-        rc = lib.gg_mipmap_warp_backward(_lib.ptr(grad_src), _lib.ptr(grad_pyr), _lib.ptr(grad_grid), go.data_ptr(),
+        grad_grid = torch.empty(g.shape, dtype=torch.float32, device=x.device) if need_g else None
+        scratch = _lib.workspace(lib.gg_mipmap_warp_backward_workspace(n, ho, wo), x.device) if (need_g and extra > 0) else None
+        rc = lib.gg_mipmap_warp_backward(_lib.ptr(grad_src), _lib.ptr(grad_pyr), _lib.ptr(grad_grid), _lib.ptr(scratch), go.data_ptr(),
                                          x.data_ptr(), _lib.ptr(pyr), g.data_ptr(), _lib.dtype_code(x), n, c, hs, ws,
                                          ho, wo, extra, max_level, min_level, pad_mode, st)
         _lib.check(rc, "gg_mipmap_warp_backward")
@@ -174,8 +175,9 @@ class _StnSample(Function):
             go = g_out.contiguous()
             if go.dtype != x.dtype:
                 go = go.to(x.dtype)
-            gg = torch.zeros(grid.shape, dtype=torch.float32, device=x.device) if need_grid else None
-            rc = lib.gg_mipmap_warp_backward(_lib.ptr(grad_src), _lib.ptr(grad_pyr), _lib.ptr(gg), go.data_ptr(), x.data_ptr(),
+            gg = torch.empty(grid.shape, dtype=torch.float32, device=x.device) if need_grid else None
+            scratch = _lib.workspace(lib.gg_mipmap_warp_backward_workspace(n, ho, wo), x.device) if (need_grid and extra > 0) else None
+            rc = lib.gg_mipmap_warp_backward(_lib.ptr(grad_src), _lib.ptr(grad_pyr), _lib.ptr(gg), _lib.ptr(scratch), go.data_ptr(), x.data_ptr(),
                                              _lib.ptr(pyr), grid.data_ptr(), _lib.dtype_code(x), n, c, hs, ws, ho, wo, extra,
                                              max_level, min_level, pad_mode, st)
             _lib.check(rc, "gg_mipmap_warp_backward")
@@ -196,10 +198,11 @@ class _StnSample(Function):
             gd = g_delta.float().contiguous() if (g_delta is not None and g_delta.dim() == 4) else None
             if (need_low or need_mask or need_theta) and (gg is not None or gd is not None):
                 g_mask = torch.empty_like(mk) if need_mask else None
-                g_low = torch.zeros_like(lo) if need_low else None
-                g_base = torch.zeros((n, 2, 3), dtype=torch.float32, device=x.device) if (need_theta and th is not None) else None
+                g_low = torch.empty_like(lo) if need_low else None
+                g_base = torch.empty((n, 2, 3), dtype=torch.float32, device=x.device) if (need_theta and th is not None) else None
                 lh, lw = lo.shape[1], lo.shape[2]
-                rc = lib.gg_flow_compose_backward(_lib.ptr(g_mask), _lib.ptr(g_low), _lib.ptr(g_base), _lib.ptr(gd), _lib.ptr(gg),
+                scratch = _lib.workspace(lib.gg_flow_compose_backward_workspace(n, lh, lw, s), x.device) if (g_low is not None or g_base is not None) else None
+                rc = lib.gg_flow_compose_backward(_lib.ptr(g_mask), _lib.ptr(g_low), _lib.ptr(g_base), _lib.ptr(scratch), _lib.ptr(gd), _lib.ptr(gg),
                                                   lo.data_ptr(), mk.data_ptr(), _lib.ptr(idn), _lib.ptr(th), _lib.ptr(al),
                                                   n, lh, lw, s, st)
                 _lib.check(rc, "gg_flow_compose_backward")

@@ -165,7 +165,10 @@ GG_API int gg_mipmap_warp_forward(void* out, float* levels_out, const void* src,
                                   const float* grid, int dtype, int64_t N, int C, int hs, int ws, int ho,
                                   int wo, int extra_levels, float max_level, float min_level,
                                   int padding_mode, void* stream);
-GG_API int gg_mipmap_warp_backward(float* grad_src, float* grad_pyramid, float* grad_grid,
+/* grad_grid is written in full; with extra_levels > 0 it needs a workspace of gg_mipmap_warp_backward_workspace
+ * bytes (the level-of-detail gradient owed to a neighbour pixel, summed in a fixed order: reproducible bits). */
+GG_API int64_t gg_mipmap_warp_backward_workspace(int64_t N, int ho, int wo);
+GG_API int gg_mipmap_warp_backward(float* grad_src, float* grad_pyramid, float* grad_grid, void* workspace,
                                    const void* grad_out, const void* src, const float* pyramid,
                                    const float* grid, int dtype, int64_t N, int C, int hs, int ws, int ho,
                                    int wo, int extra_levels, float max_level, float min_level,
@@ -184,13 +187,15 @@ GG_API int gg_warp_sample_indices(int32_t* indices, const float* grid, int64_t N
  *   low_flow (N, H, W, 2); mask (N, 9*S*S, H, W); identity_flow (S*H, S*W, 2) = F.affine_grid(identity);
  *   base_warp (N, 2, 3) or NULL; alpha (N) or NULL.  All fp32.
  *   forward : delta_flow (N, S*H, S*W, 2) and, if `flow` != NULL, flow = lerp(identity, affine(identity + delta), alpha)
- *   backward: grad_mask (written), grad_low_flow and grad_base_warp (ZERO-INITIALISED by the caller,
- *             accumulated with atomics); grad_delta / grad_flow are the incoming gradients (either may be NULL).
+ *   backward: grad_mask, grad_low_flow and grad_base_warp (each may be NULL) are written in full; the latter two need a
+ *             workspace of gg_flow_compose_backward_workspace bytes (per-pixel terms summed in a fixed order:
+ *             reproducible bits); grad_delta / grad_flow are the incoming gradients (either may be NULL).
  * ---------------------------------------------------------------------------------------------- */
 GG_API int gg_flow_compose_forward(float* delta_flow, float* flow, const float* low_flow, const float* mask,
                                    const float* identity_flow, const float* base_warp, const float* alpha,
                                    int64_t N, int H, int W, int S, void* stream);
-GG_API int gg_flow_compose_backward(float* grad_mask, float* grad_low_flow, float* grad_base_warp,
+GG_API int64_t gg_flow_compose_backward_workspace(int64_t N, int H, int W, int S);
+GG_API int gg_flow_compose_backward(float* grad_mask, float* grad_low_flow, float* grad_base_warp, void* workspace,
                                     const float* grad_delta, const float* grad_flow, const float* low_flow,
                                     const float* mask, const float* identity_flow, const float* base_warp,
                                     const float* alpha, int64_t N, int H, int W, int S, void* stream);

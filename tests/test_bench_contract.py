@@ -3,6 +3,7 @@ step on the host cores, a bounded sample: the unmodified reference code when ora
 oracle port).  Keys and invariants are the ones the driver reads."""
 import json
 import os
+import tempfile
 import subprocess
 import sys
 
@@ -43,3 +44,28 @@ def test_non_zero_ranks_of_the_reference_arm_exit_without_work():
                            "--warmup", "0"], capture_output=True, text=True, timeout=300, env=env, cwd=ROOT)
     assert proc.returncode == 0
     assert not [l for l in proc.stdout.splitlines() if l.startswith("{")]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_same_arrays_on_every_run():
+    """bench.py --dump-outputs DIR: float32 / float64 .npy files, 64 MB at most, and the same bits from two runs with the
+    same arguments."""
+    import numpy as np
+    dumps = []
+    with tempfile.TemporaryDirectory() as tmp:
+        for run in range(2):
+            out = os.path.join(tmp, "run%d" % run)
+            proc = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "0",
+                                   "--batch", "4", "--no-extra", "--no-cpu-baseline", "--dump-outputs", out],
+                                  capture_output=True, text=True, timeout=900, cwd=ROOT)
+            assert proc.returncode == 0, proc.stderr[-2000:]
+            line = json.loads(proc.stdout.strip().splitlines()[-1])
+            assert line["steps"] == 2 and line["config"]["cudnn"].startswith("deterministic")
+            files = sorted(os.listdir(out))
+            assert files == ["loss_f.npy", "loss_p.npy", "loss_tv.npy", "stn_ema_params.npy", "stn_params.npy"]
+            assert sum(os.path.getsize(os.path.join(out, f)) for f in files) <= 64 << 20
+            arrays = {f: np.load(os.path.join(out, f)) for f in files}
+            assert all(a.dtype in (np.float32, np.float64) and a.size > 0 for a in arrays.values())
+            dumps.append(arrays)
+    for f in dumps[0]:
+        assert np.array_equal(dumps[0][f], dumps[1][f]), f

@@ -5,7 +5,7 @@ import pytest
 import torch
 from torch import nn, optim
 
-from conftest import assert_close, load_golden
+from conftest import Pinned, assert_close, load_golden, state_dict_layout, zeros_state_dict
 from oracle import opset, refimport
 from oracle.make_golden import classifier_decimate, classifier_setup
 
@@ -122,13 +122,18 @@ def test_classifier_trainer_step_reports_the_reference_loss_dict_and_learns():
     assert lr0 == pytest.approx(1e-3) and ct.set_iteration(37500 // 2) == pytest.approx(0.5e-3)
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference checkout not present (container-only test)")
 def test_classifier_state_dict_is_key_compatible_with_the_reference():
-    refimport.import_reference()
-    from models import ResnetClassifier as Ref
+    """The layout (keys in order, shapes) of the reference classifier's state dict is kept in
+    tests/golden/state_dicts_classifier.npz (conftest.Pinned)."""
     from gangealing_b200.cluster_classifier import ResnetClassifier
-    r = Ref(64, channel_multiplier=0.5, num_heads=8, supersize=256)
+    pin = Pinned("state_dicts_classifier")
+
+    def reference():
+        refimport.import_reference()
+        from models import ResnetClassifier as Ref
+        return state_dict_layout(Ref(64, channel_multiplier=0.5, num_heads=8, supersize=256))
+    layout = pin.value("resnet_classifier", reference)
     m = ResnetClassifier(64, channel_multiplier=0.5, num_heads=8, supersize=256, ops=CPU)
-    assert list(r.state_dict().keys()) == list(m.state_dict().keys())
-    assert all(r.state_dict()[k].shape == m.state_dict()[k].shape for k in r.state_dict())
-    m.load_state_dict(r.state_dict())
+    assert state_dict_layout(m) == layout.tolist()
+    m.load_state_dict(zeros_state_dict(layout))
+    pin.save()

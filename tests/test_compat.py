@@ -1,15 +1,19 @@
-"""CPU, container-only: the compat shim lets the UNMODIFIED reference networks import above our op boundary
-(no import-time JIT build) and wires them to this package's ops."""
+"""CPU: the compat shim lets the UNMODIFIED reference networks import above our op boundary (no import-time JIT build)
+and wires them to this package's ops.  The reference networks come from oracle/_ref/refpy (byte-compiled by build() when
+the reference checkout is present) or from the checkout itself."""
+import os
 import subprocess
 import sys
 
 import pytest
 
 from conftest import ROOT
-from oracle import refimport
+from oracle import build_ref, refimport
+
+REFERENCE = build_ref.REFPY if build_ref.refpy_available() else refimport.REFERENCE_ROOT
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference checkout not present (container-only test)")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "models")), reason="neither oracle/_ref/refpy nor the reference checkout present")
 def test_reference_networks_import_through_the_shim():
     code = r'''
 import sys
@@ -42,6 +46,6 @@ except RuntimeError as exc:
 else:
     raise AssertionError("expected the CUDA-only boundary to refuse CPU tensors")
 print("shim ok")
-''' % (ROOT, refimport.REFERENCE_ROOT)
+''' % (ROOT, REFERENCE)
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
     assert res.returncode == 0 and "shim ok" in res.stdout, res.stdout + res.stderr

@@ -56,3 +56,27 @@ def test_apply_affine_drop_in():
     m = torch.randn(3, 2, 3, generator=g)
     grid = torch.randn(3, 9, 7, 2, generator=g)
     assert_close(stn.apply_affine(m.to(DEV), grid.to(DEV)), FL.apply_affine_ref(m, grid), rtol=1e-5)
+
+
+def test_flow_sampler_backward_is_reproducible_at_the_training_shape():
+    """The flow STN's sampling backward (grid gradient with the level-of-detail term, flow composition: low-res flow, mask,
+    similarity warp) sums in a fixed order: the same inputs give the same bits on every call, at the benchmark's shapes
+    (per-GPU batch 32, 256^2 source, 128^2 flow from 16^2 cells)."""
+    from gangealing_b200.stn import sampling as S
+    g = torch.Generator().manual_seed(3)
+    n = 32
+    img = (torch.rand(n, 3, 256, 256, generator=g) * 2 - 1).to(DEV)
+    low = (0.03 * torch.randn(n, 16, 16, 2, generator=g)).to(DEV)
+    mask = torch.randn(n, 576, 16, 16, generator=g).to(DEV)
+    theta = (torch.eye(2, 3)[None] * (0.6 + 0.8 * torch.rand(n, 1, 1, generator=g)) + 0.1 * torch.randn(n, 2, 3, generator=g)).to(DEV)
+    ident = FL.identity_flow_ref(128, 128).to(DEV)
+    go = torch.randn(n, 3, 128, 128, generator=g).to(DEV)
+
+    def grads():
+        leaves = [t.clone().requires_grad_(True) for t in (low, mask, theta)]
+        out = S.stn_sample_flow(img, leaves[0], leaves[1], ident, leaves[2], None, 8, 3.5, 0.0, "reflection")[0]
+        return torch.autograd.grad(out, leaves, go)
+    first = grads()
+    assert all(t.abs().max() > 0 for t in first)
+    for _ in range(3):
+        assert all(torch.equal(a, b) for a, b in zip(first, grads()))

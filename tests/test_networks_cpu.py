@@ -4,7 +4,7 @@ checkout is present in this container and (b) fixtures generated from them -- st
 import pytest
 import torch
 
-from conftest import assert_close, load_golden
+from conftest import Pinned, assert_close, load_golden, state_dict_layout, zeros_state_dict
 from oracle import opset, refimport
 
 CPU = opset.cpu_ops()
@@ -59,24 +59,30 @@ def test_config1_similarity_stn_64_cpu():
             assert_close(grid, blob["cfg1.grid"], rtol=1e-5)
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference checkout not present (container-only test)")
 def test_state_dicts_are_key_compatible_with_the_reference():
-    refimport.import_reference()
-    torch.Tensor.cuda = lambda self, *a, **k: self  # reference FlowHead.__init__ calls .cuda() (warping_heads.py:158)
-    from models.spatial_transformers.spatial_transformer import get_stn as ref_get_stn
-    from models.stylegan2.networks import Generator as RefG
-    from models.latent_learner import DirectionInterpolator as RefLL
+    """The layouts (keys in order, shapes) of the reference's state dicts are kept in tests/golden/state_dicts.npz
+    (conftest.Pinned)."""
+    import importlib
+    from gangealing_b200.stn import get_stn
     from gangealing_b200.training import DirectionInterpolator
-    assert list(RefG(32, 32, 2).state_dict().keys()) == list(_gen().state_dict().keys())
+    pin = Pinned("state_dicts")
+
+    def ref(module):
+        refimport.import_reference()
+        torch.Tensor.cuda = lambda self, *a, **k: self  # reference FlowHead.__init__ calls .cuda() (warping_heads.py:158)
+        return importlib.import_module(module)
+    layout = pin.value("generator", lambda: state_dict_layout(ref("models.stylegan2.networks").Generator(32, 32, 2)))
+    assert state_dict_layout(_gen()) == layout.tolist()
     for tr in (["similarity"], ["similarity", "flow"]):
-        r = ref_get_stn(list(tr), flow_size=64, supersize=128, channel_multiplier=0.5, num_heads=2)
-        from gangealing_b200.stn import get_stn
-        m = get_stn(list(tr), flow_size=64, supersize=128, channel_multiplier=0.5, num_heads=2, ops=CPU)
-        assert list(r.state_dict().keys()) == list(m.state_dict().keys())
-        m.load_state_dict(r.state_dict())
-    a = RefLL(None, 3, 5, 14, num_heads=2).state_dict()
-    b = DirectionInterpolator(None, 3, 5, 14, num_heads=2).state_dict()
-    assert list(a.keys()) == list(b.keys()) and all(a[k].shape == b[k].shape for k in a)
+        args = dict(flow_size=64, supersize=128, channel_multiplier=0.5, num_heads=2)
+        layout = pin.value("stn." + "_".join(tr), lambda: state_dict_layout(
+            ref("models.spatial_transformers.spatial_transformer").get_stn(list(tr), **args)))
+        m = get_stn(list(tr), ops=CPU, **args)
+        assert state_dict_layout(m) == layout.tolist()
+        m.load_state_dict(zeros_state_dict(layout))
+    layout = pin.value("latent_learner", lambda: state_dict_layout(ref("models.latent_learner").DirectionInterpolator(None, 3, 5, 14, num_heads=2)))
+    assert state_dict_layout(DirectionInterpolator(None, 3, 5, 14, num_heads=2)) == layout.tolist()
+    pin.save()
 
 
 def test_train_step_runs_and_learns_on_cpu_oracle_ops():

@@ -3,7 +3,7 @@ channels-last kernels vs the oracle through the C ABI (GPU)."""
 import pytest
 import torch
 
-from conftest import assert_close, golden_cases, load_golden
+from conftest import Pinned, assert_close, golden_cases, load_golden, state_dict_layout, zeros_state_dict
 from oracle.perceptual import feature_distance_ref
 
 DEV = "cuda"
@@ -68,17 +68,22 @@ def test_perceptual_module_is_key_compatible_with_the_reference_lpips():
     assert get_perceptual_loss("cpu", kind="lpips").lpips
 
 
-@pytest.mark.skipif(not __import__("oracle.refimport", fromlist=["x"]).available(), reason="reference checkout not present")
 def test_reference_lpips_state_dict_loads_into_the_mirror():
-    from oracle import refimport
-    refimport.import_reference()
-    import models.losses.lpips as L
+    """The layout of the reference LPIPS state dict is kept in tests/golden/state_dicts_lpips.npz (conftest.Pinned)."""
     from gangealing_b200.training.perceptual import PerceptualLoss
+    pin = Pinned("state_dicts_lpips")
+
+    def reference(lpips):
+        from oracle import refimport
+        refimport.import_reference()
+        import models.losses.lpips as L
+        return state_dict_layout(L.LPIPS(net="vgg", lpips=lpips, pnet_rand=True, pretrained=False, verbose=False))
     for lpips in (False, True):
-        ref = L.LPIPS(net="vgg", lpips=lpips, pnet_rand=True, pretrained=False, verbose=False)
+        layout = pin.value("lpips%d" % lpips, lambda: reference(lpips))
         ours = PerceptualLoss(lpips=lpips)
-        missing, unexpected = ours.load_state_dict(ref.state_dict(), strict=False)
+        missing, unexpected = ours.load_state_dict(zeros_state_dict(layout), strict=False)
         assert not missing and not unexpected, (missing, unexpected)
+    pin.save()
 
 
 @pytest.mark.gpu

@@ -5,6 +5,7 @@ import math
 import pytest
 import torch
 
+from conftest import Pinned
 from gangealing_b200.training import schedule as S
 from oracle import refimport
 
@@ -24,23 +25,37 @@ def test_closed_forms():
     assert s["psi"] == 0.0 and s["stn_lr"] == pytest.approx(0.5e-3) and s["ll_lr"] == pytest.approx(0.5e-2)
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference checkout not present (container-only test)")
 def test_against_the_reference_scheduler_and_annealers():
-    import importlib.util
-    import os
-    spec = importlib.util.spec_from_file_location("ref_annealing", os.path.join(refimport.REFERENCE_ROOT, "utils", "annealing.py"))
-    A = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(A)
+    """What the reference's utils/annealing.py computes is kept in tests/golden/schedule.npz (conftest.Pinned)."""
+    pin = Pinned("schedule")
+
+    def annealing():
+        import importlib.util
+        import os
+        spec = importlib.util.spec_from_file_location("ref_annealing", os.path.join(refimport.REFERENCE_ROOT, "utils", "annealing.py"))
+        A = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(A)
+        return A
     for fn in ("cosine", "linear"):
         for i in (0, 1, 777, 149999, 150000):
-            assert S.psi_at(i, 150000, fn)[0] == pytest.approx(float(A.get_psi_annealing_fn(fn)(i, 1.0, 0.0, 150000)), abs=1e-6)
-    assert S.lr_cycle_iters(150000, 37500, 1500000, 2) == A.lr_cycle_iters(150000, 37500, 1500000, 2)
-    net = torch.nn.Linear(2, 2)
-    opt = torch.optim.SGD(net.parameters(), 1e-3)
-    sched = A.DecayingCosineAnnealingWarmRestarts(opt, T_0=1, T_mult=2, decay=0.9)
-    for epoch in [0.0, 0.01, 0.5, 0.999, 1.0, 1.7, 2.99, 3.0, 6.5, 7.0, 12.345, 31.0]:
-        sched.step(epoch)
-        assert S.decaying_cosine_lr(epoch, 1e-3, 2, 0.9) == pytest.approx(opt.param_groups[0]["lr"], rel=1e-9, abs=1e-15), epoch
+            want = pin.value("psi.%s.%d" % (fn, i), lambda: float(annealing().get_psi_annealing_fn(fn)(i, 1.0, 0.0, 150000)))
+            assert S.psi_at(i, 150000, fn)[0] == pytest.approx(float(want), abs=1e-6)
+    want = pin.value("lr_cycle_iters", lambda: annealing().lr_cycle_iters(150000, 37500, 1500000, 2))
+    assert S.lr_cycle_iters(150000, 37500, 1500000, 2) == want.tolist()
+    epochs = [0.0, 0.01, 0.5, 0.999, 1.0, 1.7, 2.99, 3.0, 6.5, 7.0, 12.345, 31.0]
+
+    def reference_lrs():
+        net = torch.nn.Linear(2, 2)
+        opt = torch.optim.SGD(net.parameters(), 1e-3)
+        sched = annealing().DecayingCosineAnnealingWarmRestarts(opt, T_0=1, T_mult=2, decay=0.9)
+        lrs = []
+        for epoch in epochs:
+            sched.step(epoch)
+            lrs.append(opt.param_groups[0]["lr"])
+        return lrs
+    for epoch, lr in zip(epochs, pin.value("decaying_cosine_lr", reference_lrs).tolist(), strict=True):
+        assert S.decaying_cosine_lr(epoch, 1e-3, 2, 0.9) == pytest.approx(lr, rel=1e-9, abs=1e-15), epoch
+    pin.save()
 
 
 def test_trainer_schedule_scalars_on_cpu():

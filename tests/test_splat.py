@@ -5,7 +5,7 @@ import math
 import pytest
 import torch
 
-from conftest import assert_close
+from conftest import Pinned, assert_close
 from oracle import splat as SP
 
 DEV = "cuda"
@@ -82,29 +82,37 @@ def test_splat2d_duplicate_points_and_dense_mask():
 
 @pytest.mark.gpu
 def test_splat2d_against_the_reference_kernel():
-    """Pins both the product kernel and the oracle to the reference's own CUDA kernel on identical inputs."""
-    from oracle import build_ref
+    """Pins both the product kernel and the oracle to the reference's own CUDA kernel on identical inputs.  What the
+    reference kernel computed is kept in tests/golden/reference_splat.npz (conftest.Pinned; GG_RECORD_GOLDEN=1 with
+    oracle/_ref/ built recomputes it on the GPU)."""
     from gangealing_b200.splat2d import splat2d
-    lib = build_ref.load_splat_ref()
-    if lib is None:
-        pytest.skip("oracle/_ref/libsplat_ref.so not built (needs the reference checkout at build time)")
+    pin = Pinned("reference_splat")
     for n, p, c, h, w, sigma, soft in [(2, 800, 3, 40, 56, 0.9, False), (1, 5000, 3, 64, 64, 1.3, True)]:
         inp, coords, values, sig = _case(7 + p, n, p, c, h, w, sigma)
         d = [t.to(DEV).contiguous() for t in (inp, coords, values, sig)]
-        # host side of the reference, splat_gpu.c:20-41: zeros / clone / kernel / clamp / divide
-        alpha = torch.zeros(n, h, w, device=DEV)
-        acc = d[0].clone()
-        lib.SplatForwardGpu(torch.cuda.current_stream().cuda_stream, d[1].data_ptr(), d[2].data_ptr(), d[3].data_ptr(),
-                            alpha.data_ptr(), acc.data_ptr(), p, c, h, w, n * p)
-        torch.cuda.synchronize()
-        a = alpha.view(n, 1, h, w)
-        if soft:
-            a = a.clamp(1.0)
-        ref_out = acc / (a + 1e-8)
-        ours = splat2d(d[0], d[1], d[2], d[3], soft)
+
+        def reference():
+            from oracle import build_ref
+            lib = build_ref.load_splat_ref()
+            assert lib is not None, "oracle/_ref/libsplat_ref.so not built (python -m oracle.build_ref)"
+            # host side of the reference, splat_gpu.c:20-41: zeros / clone / kernel / clamp / divide
+            alpha = torch.zeros(n, h, w, device=DEV)
+            acc = d[0].clone()
+            lib.SplatForwardGpu(torch.cuda.current_stream().cuda_stream, d[1].data_ptr(), d[2].data_ptr(), d[3].data_ptr(),
+                                alpha.data_ptr(), acc.data_ptr(), p, c, h, w, n * p)
+            torch.cuda.synchronize()
+            a = alpha.view(n, 1, h, w)
+            if soft:
+                a = a.clamp(1.0)
+            return acc / (a + 1e-8), acc / (a + 1e-8), (alpha > 0).float()
+        got = (splat2d(d[0], d[1], d[2], d[3], soft), SP.splat2d_ref(inp, coords, values, sig, soft),
+               SP.splat2d_ref(inp, coords, values, sig, soft, return_alpha=True)[2].float())
+        (ours, ref_out), (oracle, ref_out2) = pin("case%d" % p, got[:2], lambda: reference()[:2])
+        covered, ref_covered = pin("covered%d" % p, got[2], lambda: reference()[2], keep=n * h * w)
         assert_close(ours, ref_out, rtol=1e-4, what="vs reference kernel")
-        assert_close(SP.splat2d_ref(inp, coords, values, sig, soft), ref_out, rtol=1e-4, what="oracle vs reference kernel")
-        assert torch.equal(alpha.cpu() > 0, SP.splat2d_ref(inp, coords, values, sig, soft, return_alpha=True)[2])  # same pixel set
+        assert_close(oracle, ref_out2, rtol=1e-4, what="oracle vs reference kernel")
+        assert torch.equal(covered, ref_covered)  # same pixel set
+    pin.save()
 
 
 @pytest.mark.gpu
