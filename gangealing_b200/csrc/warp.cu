@@ -806,8 +806,10 @@ int gg_mipmap_warp_forward(void* out, float* levels_out, const void* src, const 
   int rc = fill_params(&wp, N, C, hs, ws, ho, wo, padding_mode, extra_levels, max_level, min_level);
   if (rc != GG_OK) return rc;
   const int64_t total = N * ho * static_cast<int64_t>(wo);
-  if (total == 0 || C == 0) return GG_OK;
-  if (!out || !src || !grid || (extra_levels > 0 && !pyramid)) return fail(GG_ERR_BAD_ARG, "mipmap_warp_forward: null tensor");
+  if (total == 0) return GG_OK;
+  // C == 0 still writes levels_out: the level of detail depends on the grid alone (out and src are then empty)
+  if ((C > 0 && (!out || !src)) || !grid || (extra_levels > 0 && !pyramid))
+    return fail(GG_ERR_BAD_ARG, "mipmap_warp_forward: null tensor");
   auto st = static_cast<cudaStream_t>(stream);
   const int gridsz = grid_for(total, 256);
 #define GG_FWD(T_)                                                                                               \
@@ -838,8 +840,9 @@ int gg_stn_sample_forward(void* out, float* grid_out, float* delta_out, float* l
   if (rc != GG_OK) return rc;
   if (mode != 1 && mode != 2) return fail(GG_ERR_BAD_ARG, "stn_sample: mode must be 1 (affine) or 2 (flow)");
   const int64_t total = N * ho * static_cast<int64_t>(wo);
-  if (total == 0 || C == 0) return GG_OK;
-  if (!out || !src || (extra_levels > 0 && !pyramid)) return fail(GG_ERR_BAD_ARG, "stn_sample: null tensor");
+  if (total == 0) return GG_OK;
+  // C == 0 still writes grid_out, delta_out and levels_out, which do not depend on the image (out and src are then empty)
+  if ((C > 0 && (!out || !src)) || (extra_levels > 0 && !pyramid)) return fail(GG_ERR_BAD_ARG, "stn_sample: null tensor");
   if (mode == 1 && !theta) return fail(GG_ERR_BAD_ARG, "stn_sample: affine mode needs theta");
   if (mode == 2) {
     if (!low || !mask || !identity) return fail(GG_ERR_BAD_ARG, "stn_sample: flow mode needs low, mask and identity");
@@ -884,8 +887,10 @@ int gg_mipmap_warp_backward(float* grad_src, float* grad_pyramid, float* grad_gr
   int rc = fill_params(&wp, N, C, hs, ws, ho, wo, padding_mode, extra_levels, max_level, min_level);
   if (rc != GG_OK) return rc;
   const int64_t total = N * ho * static_cast<int64_t>(wo);
-  if (total == 0 || C == 0) return GG_OK;
-  if (!grad_out || !src || !grid || (extra_levels > 0 && !pyramid)) return fail(GG_ERR_BAD_ARG, "mipmap_warp_backward: null tensor");
+  if (total == 0) return GG_OK;
+  // C == 0 still writes grad_grid (zeros: no channel contributes, and no pixel owes a neighbour a level-of-detail part)
+  if ((C > 0 && (!grad_out || !src)) || !grid || (extra_levels > 0 && !pyramid))
+    return fail(GG_ERR_BAD_ARG, "mipmap_warp_backward: null tensor");
   if (grad_src && extra_levels > 0 && !grad_pyramid) return fail(GG_ERR_BAD_ARG, "mipmap_warp_backward: grad_src needs grad_pyramid");
   if (!grad_src && !grad_grid) return GG_OK;
   auto st = static_cast<cudaStream_t>(stream);

@@ -185,6 +185,76 @@ def mipmap_warp_ref(x, grid, max_num_levels=8, min_level=0.0, padding_mode="bord
     return out
 
 
+# ------------------------------------------------------------------------------------ where the gradient is decided
+# The sampler's gradient is piecewise smooth.  It jumps where a source coordinate crosses an integer (the bilinear
+# corners change), a clip bound or a reflection fold, where the level crosses an integer or a clamp, and where the
+# arg-max neighbour of the level of detail changes.  Near such a point, the last bits of an fp32 evaluation decide
+# which side is taken, so an fp32 kernel and a float64 oracle may both be right and still differ by O(1).  These
+# helpers mark the pixels where no such point is within a tolerance, measured on the oracle's own coordinates.
+def coordinate_decided(g, size, padding_mode, tol=1e-3):
+    """bool, per grid value `g` along an axis of `size` source pixels: the source coordinate is more than `tol` px from
+    an integer, from the clip bounds 0 and size-1 (border, reflection) and from the folds -1/2 and size-1/2
+    (reflection).  A coordinate clamped to a bound from more than `tol` px beyond it is decided: both sides agree."""
+    raw = ((g + 1.0) * size - 1.0) / 2.0
+    ok = torch.ones_like(raw, dtype=torch.bool)
+    pre = raw
+    if padding_mode == "reflection":
+        pre = _reflect(raw, -1, 2 * size - 1)
+        ok &= ((pre + 0.5).abs() > tol) & ((pre - (size - 0.5)).abs() > tol)
+    clamped = torch.zeros_like(ok)
+    if padding_mode != "zeros":
+        ok &= (pre.abs() > tol) & ((pre - (size - 1)).abs() > tol)
+        clamped = (pre < 0) | (pre > size - 1)
+    post = source_index(g, size, padding_mode)
+    return ok & (clamped | ((post - post.round()).abs() > tol))
+
+
+def level_decided(grid, height, width, max_num_levels, min_level=0.0, tol=1e-4, axis_ties=False):
+    """bool (N, Ho, Wo): the level of detail and the neighbour its gradient goes to are decided.
+    - the arg-max squared neighbour distance is not within `tol` of 1 (the clamp(min=1) edge);
+    - the unclamped level is more than `tol` from max_level and min_level, and, where it is not clamped, from an integer;
+    - where the level gradient flows, the largest clamped distance beats the runner-up by more than `tol` relative.
+      With `axis_ties`, a tie between left and right only, or up and down only, is allowed: on an affine grid those two
+      distances are the same function of the grid, so a reduction such as d loss / d theta does not depend on the winner
+      (a per-pixel gradient does: the part owed to the winner goes to a different pixel)."""
+    max_level = max_num_levels - 1.0
+    c = lod_coordinates(grid, height, width)
+    p = F.pad(c.permute(0, 3, 1, 2), (1, 1, 1, 1), mode="replicate").permute(0, 2, 3, 1)
+    neigh = [p[:, 1:-1, :-2], p[:, 1:-1, 2:], p[:, :-2, 1:-1], p[:, 2:, 1:-1]]  # left, right, up, down
+    sq = torch.stack([((o - c) ** 2).sum(dim=3) for o in neigh])
+    m = sq.max(dim=0).values
+    all_clamped = m < 1.0 - tol
+    raw = 0.5 * torch.log2(m.clamp(min=1.0))
+    ok = (m - 1.0).abs() > tol
+    ok &= all_clamped | (((raw - max_level).abs() > tol) & ((raw - min_level).abs() > tol))
+    flows = (~all_clamped) & (raw < max_level) & (raw > min_level)
+    ok &= ~flows | ((raw - raw.round()).abs() > tol)
+    top = sq.clamp(min=1.0).sqrt().topk(3, dim=0)
+    d, k = top.values, top.indices
+    clear = (d[0] - d[1]) > tol * d[0]
+    if axis_ties:
+        pair = torch.minimum(k[0], k[1]) * 4 + torch.maximum(k[0], k[1])
+        axis_pair = (pair == 1) | (pair == 11)                      # {left, right} or {up, down}
+        clear |= axis_pair & ((d[1] - d[2]) > tol * d[0])
+    return ok & (~flows | clear)
+
+
+def decided_pixels(grid, height, width, padding_mode="border", max_num_levels=None, min_level=0.0, coord_tol=1e-3,
+                   level_tol=1e-4, axis_ties=False):
+    """bool (N, Ho, Wo): pixels whose grid gradient is a smooth function of the grid near `grid`, for a source of
+    height x width.  The pixel's own source coordinates must be decided (coordinate_decided).  With mip levels
+    (max_num_levels not None), so must the level of detail (level_decided) of the pixel and of its four neighbours: a
+    pixel's grid gradient collects the level-of-detail parts its neighbours owe it, and their sampled values enter those
+    parts, but not their sampling derivatives."""
+    ok = coordinate_decided(grid[..., 0], width, padding_mode, coord_tol) & \
+        coordinate_decided(grid[..., 1], height, padding_mode, coord_tol)
+    if max_num_levels is None:
+        return ok
+    lod = level_decided(grid, height, width, max_num_levels, min_level, level_tol, axis_ties)
+    q = F.pad(lod[:, None].double(), (1, 1, 1, 1), mode="replicate")[:, 0] > 0.5
+    return ok & lod & q[:, 1:-1, :-2] & q[:, 1:-1, 2:] & q[:, :-2, 1:-1] & q[:, 2:, 1:-1]
+
+
 # ------------------------------------------------------------------------------------ BilinearDownsample
 def bilinear_downsample_ref(x, stride):
     """BilinearDownsample.forward (:241-256): reflect-pad stride//2, separable tent filter, stride s."""
